@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- queries/s of the gamma vector-search hot path on B200 (BASELINE.json metric).
 
-  python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME]
+  python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of nq synthetic queries: coarse quantiser,
 inverted-list scan (IVF-Flat) or LUT + ADC scan (+ exact re-rank) (IVF-PQ), top-k merge.
@@ -80,7 +80,29 @@ def parse_args():
     ap.add_argument("--profile", action="store_true",
                     help="cudaProfilerStart/Stop around the timed device steps (ncu --profile-from-start off)")
     ap.add_argument("--sweep", default="", help="nprobe:recall_num,... -> recall/QPS table on stderr, then exit")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the result of the last timed step as DIR/scores.npy (float32) and DIR/ids.npy (float64)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the result of this engine's timed step; --impl reference has none")
+    return args
+
+
+DUMP_LIMIT = 64_000_000  # bytes of .npy files --dump-outputs may write
+
+
+def dump_outputs(out_dir, scores, ids):
+    """Scores as float32, ids as float64 (exact: ids stay below 2^53).  A batch too large for DUMP_LIMIT is cut to a
+    fixed, seeded sample of its queries; their row numbers in the batch go to query_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    nq, k = scores.shape
+    row_bytes = k * (4 + 8) + 8
+    if nq * row_bytes > DUMP_LIMIT - 4096:  # 4 KiB: room for the .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(nq, (DUMP_LIMIT - 4096) // row_bytes, replace=False))
+        scores, ids = scores[rows], ids[rows]
+        np.save(os.path.join(out_dir, "query_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "scores.npy"), scores.astype(np.float32))
+    np.save(os.path.join(out_dir, "ids.npy"), ids.astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -496,13 +518,15 @@ def measure(args, wl_name, wl, n_rank, rank, world, local, use_dist, family, ste
         sync_all()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        step_device(b, timed=True)
+        last = step_device(b, timed=True)
         e1.record()
         sync_all()
         step_ms.append(e0.elapsed_time(e1))
         scan_ms.append(idx.last_scan_ms)
     if args.profile and primary:
         torch.cuda.profiler.stop()
+    # copied before the end-to-end loop below reuses the result buffers
+    outputs = (last[0].cpu().numpy(), last[1].cpu().numpy()) if args.dump_outputs and primary and rank == 0 else None
     launches = (_lib.lib().gb_launch_count() - launches0) / max(1, steps)
     stages = {kk: v / steps for kk, v in idx.stage_times().items()}
     idx.set_scan_timing(False)
@@ -567,7 +591,7 @@ def measure(args, wl_name, wl, n_rank, rank, world, local, use_dist, family, ste
     res = dict(idx=idx, wl=wl, wl_name=wl_name, params=params, build=build, nq=nq, k=k, nprobe=nprobe, recall_num=recall_num,
                sp=sp, r1=r1, r10=r10, sweep=sweep, ms_per_step=ms_per_step, scan_avg=float(np.mean(scan_ms)), launches=launches,
                stages=stages, per_rank=allr, n_total=n_total, e2e_qps=e2e_qps, cabi_qps=cabi_qps, clocks=clocks, work=work,
-               entries_all_ranks=float(ent.item()), xq_host=xq_host, family=family)
+               entries_all_ranks=float(ent.item()), xq_host=xq_host, family=family, outputs=outputs)
     return res
 
 
@@ -694,6 +718,8 @@ def main():
             "gpu_launches": res["launches"],
             "roofline": roofline,
             "cpu_baseline": cpu}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *res["outputs"])
     idx.close()
     del res
 
