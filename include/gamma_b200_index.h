@@ -136,6 +136,12 @@ int gb_index_search_preassigned(gb_index *index, int nq, const float *x, int k, 
                                 float min_score, float max_score, float *out_scores, int64_t *out_ids);
 /* pq.compute_codes on residuals (gamma_index_ivfpq.cc:489-494) */
 int gb_index_pq_encode(gb_index *index, int64_t n, const float *x, const int64_t *assign, uint8_t *codes);
+/* IVFRABITQ: rabitq.compute_codes_core on residuals (gamma_index_ivfrabitq.cc:304-418), codes n x code_size */
+int gb_index_rabitq_encode(gb_index *index, int64_t n, const float *x, const int64_t *assign, uint8_t *codes);
+/* IVFRABITQ test hook: the scan's per-(query, probe) constants, out = nq x nprobe x 8 floats
+ * {vl, delta, cB*sum qq, cB*d, |q-c|^2 (L2) or <q,c> (IP), 1.9 |q-c|, sum qq (int32 bits), cB} (DESIGN.md section 5b) */
+int gb_index_rabitq_query_consts(gb_index *index, int nq, const float *x, const int64_t *keys, int nprobe, int qb,
+                                 int centered, float *out);
 
 /* ---- standalone kernels exposed for tests / bench ---- */
 /* faiss Clustering restated (k-means), host in/out; obj (niter floats) may be NULL */

@@ -84,6 +84,8 @@ def _declare(l):
     l.gb_index_coarse_search.argtypes = [vp, i32, vp, i32, vp, vp]
     l.gb_index_search_preassigned.argtypes = [vp, i32, vp, i32, vp, vp, i32, cstr, vp, vp, i64, f32, f32, vp, vp]
     l.gb_index_pq_encode.argtypes = [vp, i64, vp, vp, vp]
+    l.gb_index_rabitq_encode.argtypes = [vp, i64, vp, vp, vp]
+    l.gb_index_rabitq_query_consts.argtypes = [vp, i32, vp, vp, i32, i32, i32, vp]
     l.gb_kmeans.argtypes = [i32, vp, i64, i32, i32, i32, i64, i32, i32, vp, vp]
     l.gb_kmeans_update.argtypes = [i32, vp, i64, i32, i32, vp, vp]
     l.gb_merge_partitions_device.argtypes = [i32, vp, vp, i32, i32, i32, i32, vp, vp, vp]

@@ -317,7 +317,8 @@ Status Engine::CreateTable(const uint8_t* fb, size_t len) {
     training_threshold_ = mp.training_threshold;  // table.cc:143-150
   if (training_threshold_ > 0) mp.training_threshold = training_threshold_;
   Index* idx = create_index(index_type_, dim_, mp, device_, 20);
-  if (!idx) return Status::Make(index_type_ == "FLAT" || index_type_ == "IVFFLAT" || index_type_ == "IVFPQ"
+  if (!idx) return Status::Make(index_type_ == "FLAT" || index_type_ == "IVFFLAT" || index_type_ == "IVFPQ" ||
+                                        index_type_ == "IVFRABITQ"
                                     ? kInvalidArgument
                                     : kNotSupported,
                                 last_error());

@@ -153,6 +153,8 @@ struct ModelParams {  // index/impl/gamma_index_ivfpq.h:1031-1257, gamma_index_i
   int bucket_init_size = 1000;
   int bucket_max_size = 1280000;
   int opq_nsubvector = 0;       // > 0: OPQ rotation in front of the IVFPQ index (gamma_index_ivfpq.h:1202-1216)
+  int nb_bits = 4;              // IVFRABITQ bits per dimension, [1, 9] (gamma_index_ivfrabitq.h:335-537)
+  int qb = 4;                   // IVFRABITQ query bits, [0, 8]; 0 = float query
 };
 
 struct RetrievalParams {  // gamma_index_ivfpq.cc:233-294, gamma_index_ivfflat.cc:293-340
@@ -161,6 +163,8 @@ struct RetrievalParams {  // gamma_index_ivfpq.cc:233-294, gamma_index_ivfflat.c
   int recall_num = -1;
   int parallel_on_queries = 1;
   bool brute_force = false;
+  int qb = -1;            // IVFRABITQ: query bits for this search; outside [0, 8] => the model's qb
+  bool centered = false;  // IVFRABITQ: quantise the query on a grid symmetric around zero
 };
 
 struct SearchContext {  // RetrievalContext / SearchCondition (common/gamma_common_data.h:33-121)
@@ -479,6 +483,31 @@ class IVFPQIndex : public IVFFlatIndex {
   int set_opq(const float* host_A);        // d x d row-major; marks the rotation trained
   int get_opq(float* host_A) const;
   int apply_opq_host(const float* x, int64_t n, float* out);  // test hook: y = A x through the device path
+};
+
+// IVF with RaBitQ codes of the residuals (faiss IndexIVFRaBitQ behind gamma_index_ivfrabitq.{h,cc}); everything but
+// the codec and the scan is the IVF-Flat machinery.  Scores: the full nb_bits estimate of every valid entry in the probed
+// lists (DESIGN.md section 5b), optionally re-ranked exactly (recall_num).
+class IVFRaBitQIndex : public IVFFlatIndex {
+ public:
+  IVFRaBitQIndex(int d, const ModelParams& mp, int device, int seg_shift);
+  int training_threshold() const override;
+  int nb_bits() const { return mp_.nb_bits; }
+  int encode_host(const float* x, int64_t n, const int64_t* assign, uint8_t* codes_out);
+  // test hook: the per-pair constants (nq x nprobe x kRabitqConsts) the scan uses
+  int query_consts_host(int nq, const float* x, const int64_t* keys, int nprobe, int qb, bool centered, float* out);
+  int resolve_qb(const SearchContext& ctx) const;
+
+ protected:
+  int code_bytes() const override { return rabitq_code_size(d_, mp_.nb_bits); }
+  const char* gamma_file_name() const override;
+  int dump_gamma_extra(FILE* f) override;
+  int load_gamma_extra(FILE* f) override;
+  int append_batch(const float* x, int64_t n, int64_t vid0, const int32_t* d_list, const int32_t* d_pos,
+                   const int32_t* d_assign, Scratch& s) override;
+  int scan_dev(const SearchContext& ctx, const FilterArgs& f, int metric, int nq, const float* xq, int k,
+               const int32_t* probe_ids, const float* coarse_dis, int nprobe, unsigned long long* out_keys,
+               Scratch& s) override;
 };
 
 // reflector (index/reflector.h:68-80): type name -> index object

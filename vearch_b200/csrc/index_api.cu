@@ -84,6 +84,21 @@ bool parse_model_params(const std::string& text, ModelParams* mp, std::string* e
     if (v > 0) mp->bucket_max_size = v;
   }
   if (jv.get_int("training_threshold", &v) && v > 0) mp->training_threshold = v;
+  // IVFRABITQ (gamma_index_ivfrabitq.h:335-537): kept as given, range-checked by create_index("IVFRABITQ")
+  if (jv.get("nb_bits")) {
+    if (!jv.get_int("nb_bits", &v)) {
+      *err = "invalid nb_bits should be integer in [1, 9]";
+      return false;
+    }
+    mp->nb_bits = v;
+  }
+  if (jv.get("qb")) {
+    if (!jv.get_int("qb", &v)) {
+      *err = "invalid qb should be integer in [0, 8]";
+      return false;
+    }
+    mp->qb = v;
+  }
   std::string mt;
   if (jv.get_string("metric_type", &mt)) {
     if (strcasecmp("L2", mt.c_str()) && strcasecmp("InnerProduct", mt.c_str())) {
@@ -110,6 +125,9 @@ bool parse_retrieval_params(const std::string& text, RetrievalParams* rp, std::s
   if (jv.get_int("recall_num", &v) && v > 0) rp->recall_num = v;
   if (jv.get_int("nprobe", &v) && v > 0) rp->nprobe = v;
   if (jv.get_int("parallel_on_queries", &v)) rp->parallel_on_queries = v != 0;
+  if (jv.get_int("qb", &v)) rp->qb = v < 0 ? -2 : v;  // IVFRABITQ; out of range => the model's qb
+  bool b;
+  if (jv.get_bool("centered", &b)) rp->centered = b;
   return true;
 }
 
@@ -281,6 +299,10 @@ static IVFPQIndex* as_pq(gb_index* index) {
   if (!index || !index->impl) return nullptr;
   return dynamic_cast<IVFPQIndex*>(index->impl);
 }
+static IVFRaBitQIndex* as_rq(gb_index* index) {
+  if (!index || !index->impl) return nullptr;
+  return dynamic_cast<IVFRaBitQIndex*>(index->impl);
+}
 #define IVF_OR_FAIL(v, index)                \
   IVFFlatIndex* v = as_ivf(index);           \
   if (!v) {                                  \
@@ -372,6 +394,7 @@ int gb_index_list_len(gb_index* index, int list) {
 int gb_index_code_size(gb_index* index) {
   IVF_OR_FAIL(ivf, index);
   IVFPQIndex* pq = as_pq(index);
+  if (IVFRaBitQIndex* rq = as_rq(index)) return rabitq_code_size(rq->d(), rq->nb_bits());
   return pq ? pq->M() : ((ivf->d() + 3) / 4 * 4) * 4;
 }
 int gb_index_get_list(gb_index* index, int list, uint8_t* codes, int64_t* ids) {
@@ -403,6 +426,23 @@ int gb_index_search_preassigned(gb_index* index, int nq, const float* x, int k, 
   SearchContext ctx;
   if (fill_ctx(&ctx, retrieval_params_json, 0, del_bitmap, filter_bitmap, bitmap_bits, min_score, max_score)) return -1;
   return ivf->search_preassigned_host(ctx, nq, x, k, keys, coarse_dis, nprobe, out_scores, out_ids);
+}
+int gb_index_rabitq_encode(gb_index* index, int64_t n, const float* x, const int64_t* assign, uint8_t* codes) {
+  IVFRaBitQIndex* rq = as_rq(index);
+  if (!rq) {
+    set_last_error("not an IVFRABITQ index");
+    return -1;
+  }
+  return rq->encode_host(x, n, assign, codes);
+}
+int gb_index_rabitq_query_consts(gb_index* index, int nq, const float* x, const int64_t* keys, int nprobe, int qb,
+                                 int centered, float* out) {
+  IVFRaBitQIndex* rq = as_rq(index);
+  if (!rq) {
+    set_last_error("not an IVFRABITQ index");
+    return -1;
+  }
+  return rq->query_consts_host(nq, x, keys, nprobe, qb, centered != 0, out);
 }
 int gb_index_pq_encode(gb_index* index, int64_t n, const float* x, const int64_t* assign, uint8_t* codes) {
   PQ_OR_FAIL(pq, index);

@@ -194,6 +194,31 @@ cudaError_t launch_rerank(const unsigned long long* cand_keys, int ncand, int nq
                           const float* const* raw_segments, int seg_shift, int64_t ld_raw, int k, int metric,
                           FilterArgs f, unsigned long long* out_keys, cudaStream_t st);
 
+// ---- IVFRABITQ: RaBitQ codes, query quantisation, scan (kernels_rabitq.cu; DESIGN.md section 5b) ---------
+// bytes per entry: sign plane (P = ceil(d/8)) + {or_c, f1} (1 bit) or
+// sign plane + {or_c, f1, f_error} + (nb_bits - 1) extra planes + {f_ex} (multi-bit)
+__host__ __device__ inline int rabitq_code_size(int d, int nb_bits) {
+  const int P = (d + 7) / 8;
+  return nb_bits == 1 ? P + 8 : nb_bits * P + 16;
+}
+// per-(query, probe) constants: {vl, delta, cB * sum qq, cB * d, |q-c|^2 (L2) / <q,c> (IP), 1.9 |q-c|, sum qq (int bits), cB}
+constexpr int kRabitqConsts = 8;
+// codes[i] = code of x_i - coarse[assign_i] (assign < 0: centroid 0, the row is not appended)
+cudaError_t launch_rabitq_encode(const float* x, int64_t ldx, int64_t n, int d, const float* coarse, int64_t ldc,
+                                 const int32_t* assign, int nb_bits, int metric, uint8_t* codes, cudaStream_t st);
+// pair j = q * nprobe + p: consts[j][8], planes[j][qb][ceil(d/32)] (qb > 0)
+cudaError_t launch_rabitq_query_prep(const float* xq, int64_t ldq, int nq, int d, const int32_t* probe_ids, int nprobe,
+                                     const float* coarse, int64_t ldc, int nlist, int qb, bool centered, int nb_bits,
+                                     int metric, float* consts, uint32_t* planes, cudaStream_t st);
+// partial[q][group][k] sorted keys, group = ceil(nprobe / pg) CTAs per query (pg <= 32)
+// false if the scan's shared-memory ring (two stages of at least 16 codes) cannot hold codes of this shape
+bool rabitq_scan_supported(int d, int nb_bits);
+// (qb = 0: the float query residual x_q - c is formed in the scan from xq and coarse)
+cudaError_t launch_rabitq_scan(const float* consts, const uint32_t* planes, const float* xq, int64_t ldq,
+                               const float* coarse, int64_t ldc, int nq,
+                               const int32_t* probe_ids, int nprobe, int pg, ListDirectory dir, int d, int nb_bits, int qb,
+                               int k, int metric, FilterArgs f, unsigned long long* partial, cudaStream_t st);
+
 // ---- K6/K8: build-side kernels ------------------------------------------------------------
 // centroids[c] = (sum of x[perm[off[c]..off[c+1])] in that order) * (1/count); empty => zeros
 cudaError_t launch_segment_mean(const float* x, int64_t ldx, int d, const int32_t* perm, const int32_t* off, int k,

@@ -334,6 +334,24 @@ class GammaIndex:
         _check(_lib.lib().gb_index_pq_encode(self._h, x.shape[0], _ptr(x), _ptr(assign), _ptr(codes)), "pq_encode")
         return codes
 
+    def rabitq_encode(self, x, assign):
+        """IVFRABITQ: RaBitQ codes (n x code_size uint8) of x against centroids[assign], on the device."""
+        x = _f32(x)
+        assign = np.ascontiguousarray(assign, np.int64)
+        codes = np.empty((x.shape[0], self.code_size), np.uint8)
+        _check(_lib.lib().gb_index_rabitq_encode(self._h, x.shape[0], _ptr(x), _ptr(assign), _ptr(codes)), "rabitq_encode")
+        return codes
+
+    def rabitq_query_consts(self, x, keys, qb, centered=False):
+        """IVFRABITQ: the scan's per-(query, probe) constants, [nq, nprobe, 8] float32 (DESIGN.md section 5b)."""
+        x = _f32(x)
+        keys = np.ascontiguousarray(keys, np.int64)
+        nq, nprobe = keys.shape
+        out = np.empty((nq, nprobe, 8), np.float32)
+        _check(_lib.lib().gb_index_rabitq_query_consts(self._h, nq, _ptr(x), _ptr(keys), nprobe, qb, int(centered), _ptr(out)),
+               "rabitq_query_consts")
+        return out
+
 
 def index_factory(d, description, metric=METRIC_L2, device=0, **extra):
     """index/index.h index_factory: "IVF1024,Flat" | "IVF4096,PQ16x8" | "Flat"."""
